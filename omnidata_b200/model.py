@@ -21,7 +21,7 @@ import torch
 import torch.nn as nn
 import torch.nn.functional as F
 
-from . import ops
+from . import bwd, ops
 from ._capi import OdbError
 
 _STAGES = ((256, 3), (512, 4), (1024, 9))   # timm ResNetV2(layers=(3,4,9)) widths / depths
@@ -185,18 +185,20 @@ def _std_weight(w: torch.Tensor, eps: float = 1e-8) -> torch.Tensor:
 
 
 class _Workspace:
-    """Named device buffers for one (batch, height, width); allocated once, reused every forward."""
+    """Named device buffers, allocated once and reused every forward; a name asked for with another shape (a tuple or
+    torch.Size) or dtype gets a new buffer."""
 
     def __init__(self, device):
         self.device = device
-        self.bufs: Dict[str, torch.Tensor] = {}
+        # name -> (buffer, shape, dtype) as requested: comparing those costs less host time than reading t.shape
+        self._bufs: Dict[str, tuple] = {}
 
-    def get(self, name: str, shape, dtype=torch.bfloat16) -> torch.Tensor:
-        t = self.bufs.get(name)
-        if t is None:
-            t = torch.empty(tuple(shape), device=self.device, dtype=dtype)
-            self.bufs[name] = t
-        return t
+    def get(self, name: str, shape, dtype=torch.bfloat16, zero: bool = False) -> torch.Tensor:
+        e = self._bufs.get(name)
+        if e is None or e[1] != shape or e[2] is not dtype:
+            alloc = torch.zeros if zero else torch.empty
+            e = self._bufs[name] = (alloc(shape, device=self.device, dtype=dtype), shape, dtype)
+        return e[0]
 
 
 class DPTDepthModel(nn.Module):
@@ -451,80 +453,6 @@ class DPTDepthModel(nn.Module):
         graph.replay()
         return static_out.clone()
 
-    def _resnet_features(self, x, pk, ws, taps):
-        """ResNetV2 stem + stages of the hybrid encoder -> (layer_1, layer_2, stage-2 features)."""
-        B, _, H, W = x.shape
-        fp32 = self._precision == "fp32"
-        adt = torch.float32 if fp32 else torch.bfloat16
-        buf = lambda name, shape, dtype=None: ws.get(name, shape, adt if dtype is None else dtype)
-        # ---------------- ResNetV2 stem + stages (timm; hooks at vit.py:363-368)
-        h2, w2 = H // 2, W // 2
-        n_gn = 1 + sum(3 * d + 1 for _, d in _STAGES)
-        stats_pool = buf("gn_stats", (n_gn, B, 32, 2), torch.float32)
-        gn_scratch = ws.bufs.get("gn_scratch")
-        if gn_scratch is None:                         # zeroed once; the kernel leaves it zeroed
-            gn_scratch = ws.bufs["gn_scratch"] = torch.zeros(4 << 20, dtype=torch.uint8, device=x.device)
-        stat_i = iter(range(n_gn))
-        # fused statistics: the conv epilogue writes per-warp partial sums here (largest layer:
-        # stage 0 at 96x96 -> 72 tiles x 4 quadrants x 32 groups x 2 per image)
-        gn_part = buf("gn_partial", (B * ((H // 4) * (W // 4) // 32 + 64) * 4 * 32 * 2,), torch.float32)
-
-        def conv_stats(fn, *args, out, **kw):
-            """conv + GroupNorm statistics of its (unrounded) output.  Tensor-core path: partial sums in the conv
-            epilogue + finalize; fp32 mode: the deterministic standalone statistics kernel."""
-            st = stats_pool[next(stat_i)]
-            if fp32:
-                fn(*args, out, **kw)
-                ops.groupnorm_stats(out, st, scratch=gn_scratch)
-            else:
-                fn(*args, out, gn_stats=(gn_part, st), **kw)
-            return st
-
-        cols = buf("stem_cols", (B * h2 * w2, 160))
-        ops.stem_im2col(x, cols)
-        s0 = buf("stem_conv", (B, h2, w2, 64))
-        st = conv_stats(ops.conv1x1, cols.view(B, h2, w2, 160), pk["stem_w"], out=s0)
-        t = buf("stem_pool", (B, h2 // 2, w2 // 2, 64))
-        ops.stem_gn_relu_maxpool(s0, st, pk["stem_g"], pk["stem_b"], t)
-        if taps is not None:
-            taps["stem_conv"], taps["stem_pool"] = s0, t
-        feats = []
-        hh, ww = h2 // 2, w2 // 2
-        for s, b, e in pk["rn_blocks"]:
-            stride, cout, mid = e["stride"], e["cout"], e["mid"]
-            ho, wo = hh // stride, ww // stride
-            tag = f"s{s}b{b}"
-            shortcut, sc_stats = t, None
-            if b == 0:
-                d = buf(tag + "_ds", (B, ho, wo, cout))
-                sc_stats = conv_stats(ops.conv1x1, t[:, ::stride, ::stride, :] if stride > 1 else t, e["wd"], out=d)
-                shortcut = d
-            y1 = buf(tag + "_y1", (B, hh, ww, mid))
-            st1 = conv_stats(ops.conv1x1, t, e["w1"], out=y1)
-            a1 = buf(tag + "_a1", (B, hh, ww, mid))
-            ops.groupnorm_apply(y1, st1, e["g1"], e["b1"], a1, relu=True)
-            y2 = buf(tag + "_y2", (B, ho, wo, mid))
-            if stride == 1:
-                st2 = conv_stats(ops.conv3x3, a1, e["w2"], out=y2)
-            else:
-                st2 = conv_stats(lambda a, w_, o, **kw: ops.conv3x3_s2(a, w_, o, "same", **kw), a1, e["w2"], out=y2)
-            a2 = buf(tag + "_a2", (B, ho, wo, mid))
-            ops.groupnorm_apply(y2, st2, e["g2"], e["b2"], a2, relu=True)
-            y3 = buf(tag + "_y3", (B, ho, wo, cout))
-            st3 = conv_stats(ops.conv1x1, a2, e["w3"], out=y3)
-            out = buf(tag + "_out", (B, ho, wo, cout))
-            if b == 0:
-                ops.groupnorm_apply(y3, st3, e["g3"], e["b3"], out, relu=True, res=shortcut,
-                                    res_stats=sc_stats, res_gamma=e["gd"], res_beta=e["bd"])
-            else:
-                ops.groupnorm_apply(y3, st3, e["g3"], e["b3"], out, relu=True, res=shortcut)
-            t, hh, ww = out, ho, wo
-            if taps is not None:
-                taps[f"{tag}_out"] = out
-            if b == _STAGES[s][1] - 1:
-                feats.append(t)
-        return feats
-
     @torch.no_grad()
     def _forward_impl(self, x: torch.Tensor) -> torch.Tensor:
         pk = self._packed
@@ -536,177 +464,327 @@ class DPTDepthModel(nn.Module):
         taps = self.taps if self.keep_taps else None
         if taps is not None:
             taps.clear()
-        fp32 = self._precision == "fp32"
-        adt = torch.float32 if fp32 else torch.bfloat16            # activation storage type
-        buf = lambda name, shape, dtype=None: ws.get(name, shape, adt if dtype is None else dtype)
-
-        D, heads = self.arch["embed"], self.arch["heads"]
-        hooks = self.arch["hooks"]
-        if self.arch["hybrid"]:
-            layer_1, layer_2, f3 = self._resnet_features(x, pk, ws, taps)
-            gh, gw = f3.shape[1], f3.shape[2]
-        else:
-            gh, gw = H // 16, W // 16
-        ntok = gh * gw + 1
-
-        # ---------------- tokens: patch proj + cls + pos (vit.py:131-147).  The residual stream is fp32 in BOTH
-        # precisions (timm Block.forward adds every branch to an fp32 `x`; SURVEY.md C.1): the proj / fc2 epilogues
-        # read and write fp32, LayerNorm reads fp32.
+        gh, gw = H // 16, W // 16
         pos0, pos_grid = self._pos_for_grid(pk, gh, gw)
         pos_b = pk["pos_cache"].get((gh, gw, B))           # derived from the weights: lives with the packed weights
         if pos_b is None:                                  # pos[1:] replicated per image: the GEMM's fp32 residual operand
             pos_b = pk["pos_cache"][(gh, gw, B)] = pos_grid.unsqueeze(0).expand(B, -1, -1).contiguous()
-        tok_bufs = [buf(f"tok_{i}", (B, ntok, D), torch.float32) for i in range(len(hooks))]
-        tok = tok_bufs[0]
-        ops.write_cls_row(tok, pk["cls"], pos0)
-        if self.arch["hybrid"]:
-            ops.linear(f3.view(B, 1, gh * gw, 1024), pk["proj_w"], tok[:, 1:, :].unsqueeze(1), bias=pk["proj_b"],
-                       residual=pos_b.unsqueeze(1))
-        else:
-            cols = buf("patch_cols", (B, 1, gh * gw, 3 * 16 * 16))
-            ops.patchify(x, cols.view(B * gh * gw, -1), 16)
-            ops.linear(cols, pk["proj_w"], tok[:, 1:, :].unsqueeze(1), bias=pk["proj_b"], residual=pos_b.unsqueeze(1))
-
+        out = network_forward(pk, x, ws, self.arch, self._precision == "fp32", (pos0, pos_b), self.non_negative, taps=taps)
         if taps is not None:
-            taps["tokens_in"] = tok.clone()
-        # ---------------- ViT blocks (vit.py:150-151); final norm is dead compute and skipped.  The residual
-        # stream lives in one buffer per hooked block: the block after a hook writes its first residual add
-        # into the next buffer, which leaves the hooked activation intact.
-        hbuf = buf("vit_h", (B, ntok, D))
-        qkv = buf("vit_qkv", (B, ntok, 3 * D))
-        att = buf("vit_att", (B, ntok, D))
-        mlp = buf("vit_mlp", (B, ntok, 4 * D))
-        rows = B * ntok
-        cur = tok
-        hooked = []
-        for i, blk in enumerate(pk["vit"]):
-            ops.layernorm(cur, blk["ln1"][0], blk["ln1"][1], hbuf)
-            ops.linear(hbuf.view(rows, -1), blk["qkv"][0], qkv.view(rows, -1), bias=blk["qkv"][1])
-            ops.attention(qkv, att, heads=heads, scale=0.125)
-            nxt = tok_bufs[len(hooked)] if (i - 1) in hooks else cur
-            ops.linear(att.view(rows, -1), blk["proj"][0], nxt.view(rows, -1), bias=blk["proj"][1],
-                       residual=cur.view(rows, -1))
-            cur = nxt
-            ops.layernorm(cur, blk["ln2"][0], blk["ln2"][1], hbuf)
-            ops.linear(hbuf.view(rows, -1), blk["fc1"][0], mlp.view(rows, -1), bias=blk["fc1"][1],
-                       act=ops.ACT_GELU)
-            ops.linear(mlp.view(rows, -1), blk["fc2"][0], cur.view(rows, -1), bias=blk["fc2"][1],
-                       residual=cur.view(rows, -1))
-            if i in hooks:
-                hooked.append(cur)
-            if taps is not None:
-                taps[f"tokens_{i}"] = cur.clone()
-
-        # ---------------- reassemble (vit.py:66-97, 185-290 / 431-462)
-        def readout(tk, n, cout):
-            if not fp32:                                   # the hooked activation leaves the fp32 stream as a bf16 operand
-                tk16 = buf(f"ro{n}_tok", (B, ntok, D))
-                ops.cast_f32_bf16(tk, tk16)
-                tk = tk16
-            cb = buf(f"ro{n}_cb", (B, D), torch.float32)
-            ops.readout_cls_bias(pk[f"ro{n}_wfull"], pk[f"ro{n}_b"], tk, cb)
-            r = buf(f"ro{n}_r", (B, 1, gh * gw, D))
-            ops.linear(tk[:, 1:, :].unsqueeze(1), pk[f"ro{n}_wtok"], r, bias=cb, bias_per_image=True,
-                       act=ops.ACT_GELU)
-            o = buf(f"pp{n}", (B, gh, gw, cout))
-            ops.conv1x1(r.view(B, gh, gw, D), pk[f"pp{n}_w"], o, bias=pk[f"pp{n}_b"])
-            return o
-
-        def conv_transpose(t, n, k):
-            """ConvTranspose2d(c, c, k, stride k): phase (dy, dx) of the output is a 1x1 convolution of the
-            input, stored through a strided view of the output (no scatter kernel)."""
-            c = t.shape[3]
-            o = buf(f"pp{n}t", (B, gh * k, gw * k, c))
-            for dy in range(k):
-                for dx in range(k):
-                    ops.conv1x1(t, pk[f"pp{n}t_w"][dy][dx], o[:, dy::k, dx::k, :], bias=pk[f"pp{n}t_b"])
-            return o
-
-        rn_in = self._rn_pad                 # (reassemble widths, zero-padded to the GEMM's N granularity)
-        if self.arch["hybrid"]:
-            tokens_8, tokens_11 = hooked
-            layer_3 = readout(tokens_8, 3, rn_in[2])
-            u4 = readout(tokens_11, 4, rn_in[3])
-        else:
-            layer_1 = conv_transpose(readout(hooked[0], 1, rn_in[0]), 1, 4)
-            layer_2 = conv_transpose(readout(hooked[1], 2, rn_in[1]), 2, 2)
-            layer_3 = readout(hooked[2], 3, rn_in[2])
-            u4 = readout(hooked[3], 4, rn_in[3])
-        layer_4 = buf("pp4s", (B, gh // 2, gw // 2, rn_in[3]))
-        ops.conv3x3_s2(u4, pk["pp4s_w"], layer_4, "sym1", bias=pk["pp4s_b"])
-
-        # ---------------- scratch.layerN_rn (dpt_depth.py:73-76): raw + relu copies feed the RCUs
-        rn_raw, rn_relu = [], []
-        for n, l in zip((1, 2, 3, 4), (layer_1, layer_2, layer_3, layer_4)):
-            shp = (B, l.shape[1], l.shape[2], _FEATURES)
-            raw, rl = buf(f"rn{n}_raw", shp), buf(f"rn{n}_relu", shp)
-            ops.conv3x3(l, pk[f"rn{n}_w"], raw, out2=rl)
-            rn_raw.append(raw)
-            rn_relu.append(rl)
-
-        # ---------------- RefineNet fusion (dpt_depth.py:78-81; blocks.py:263-341)
-        def rcu(n, u, x_raw, x_relu, out, out2=None):
-            (w1, b1), (w2, b2) = pk[f"ff{n}_rcu{u}"]
-            tmid = buf(f"ff{n}_rcu{u}_t", x_raw.shape)
-            ops.conv3x3(x_relu, w1, tmid, bias=b1, act=ops.ACT_RELU)       # relu(conv1(relu(x)))
-            ops.conv3x3(tmid, w2, out, bias=b2, residual=x_raw, out2=out2)  # conv2(.) + x
-
-        def fusion_tail(n, s_raw, s_relu):
-            """RCU2, then the 1x1 out_conv at the input resolution (it commutes with the bilinear
-            upsample: the interpolation weights sum to one)."""
-            y = buf(f"ff{n}_y", s_raw.shape)
-            rcu(n, 2, s_raw, s_relu, y)
-            z = buf(f"ff{n}_z", s_raw.shape)
-            w, bias = pk[f"ff{n}_out"]
-            ops.conv1x1(y, w, z, bias=bias)
-            return z
-
-        z = fusion_tail(4, rn_raw[3], rn_relu[3])
-        if taps is not None:
-            taps["path_4"] = self._debug_upsample(z)
-        for n in (3, 2, 1):
-            l_raw, l_relu = rn_raw[n - 1], rn_relu[n - 1]
-            res = buf(f"ff{n}_res", l_raw.shape)
-            rcu(n, 1, l_raw, l_relu, res)
-            s_raw, s_relu = buf(f"ff{n}_s", l_raw.shape), buf(f"ff{n}_s_relu", l_raw.shape)
-            ops.upsample2x_add(z, s_raw, res=res, out_relu=s_relu)         # up(path) + RCU1(layer_rn)
-            z = fusion_tail(n, s_raw, s_relu)
-            if taps is not None and n > 1:
-                taps[f"path_{n}"] = self._debug_upsample(z)
-        path_1 = buf("path_1", (B, z.shape[1] * 2, z.shape[2] * 2, _FEATURES))
-        ops.upsample2x_add(z, path_1)
-
-        # ---------------- head (dpt_depth.py:91-99)
-        w0, b0 = pk["head0"]
-        h1 = buf("head_h1", (B, path_1.shape[1], path_1.shape[2], _FEATURES // 2))
-        ops.conv3x3(path_1, w0, h1, bias=b0)
-        h1u = buf("head_h1u", (B, H, W, _FEATURES // 2))
-        ops.upsample2x_add(h1, h1u)
-        out = buf("out", (B, self.num_channels, H, W), torch.float32)
-        w2, b2 = pk["head2"]
-        w4, b4 = pk["head4"]
-        if fp32:
-            # correctness mode: the 128 -> 32 conv (+ReLU) on the FP32 pipe, then the 1x1 conv (+ReLU) to NCHW
-            h2 = buf("head_h2", (B, H, W, 32))
-            ops.conv3x3(h1u, w2, h2, bias=b2, act=ops.ACT_RELU)
-            pre = buf("head_pre", (B, self.num_channels, H, W), torch.float32) if taps is not None else None
-            ops.head_tail_f32(h2, w4, b4, out, relu=self.non_negative, pre=pre)
-            if taps is not None:
-                taps["head_pre_relu"] = pre
-        else:
-            ops.conv3x3(h1u, w2, None, bias=b2, head=(w4, b4, out, self.non_negative))
-
-        if taps is not None:
-            for hk, tk in zip(hooks, hooked):
-                taps[f"tokens_{hk}"] = tk
-            taps.update(layer_1=layer_1, layer_2=layer_2, layer_3=layer_3, layer_4=layer_4, path_1=path_1,
-                        layer_1_rn=rn_raw[0], layer_2_rn=rn_raw[1], layer_3_rn=rn_raw[2],
-                        layer_4_rn=rn_raw[3])
             self.taps = {k: v.clone() for k, v in taps.items()}
         return out if (self.use_cuda_graph and not self.keep_taps) else out.clone()
 
-    @staticmethod
-    def _debug_upsample(z: torch.Tensor) -> torch.Tensor:
-        o = torch.empty((z.shape[0], 2 * z.shape[1], 2 * z.shape[2], z.shape[3]), device=z.device, dtype=z.dtype)
-        ops.upsample2x_add(z, o)
+
+def _debug_upsample(z: torch.Tensor) -> torch.Tensor:
+    o = torch.empty((z.shape[0], 2 * z.shape[1], 2 * z.shape[2], z.shape[3]), device=z.device, dtype=z.dtype)
+    ops.upsample2x_add(z, o)
+    return o
+
+
+def _resnet_features(pk, x, ws, fp32, taps, save):
+    """ResNetV2 stem + stages of the hybrid encoder -> (layer_1, layer_2, stage-2 features)."""
+    B, _, H, W = x.shape
+    adt = torch.float32 if fp32 else torch.bfloat16
+    buf = lambda name, shape, dtype=adt: ws.get(name, shape, dtype)
+    # ---------------- ResNetV2 stem + stages (timm; hooks at vit.py:363-368)
+    h2, w2 = H // 2, W // 2
+    n_gn = 1 + sum(3 * d + 1 for _, d in _STAGES)
+    stats_pool = buf("gn_stats", (n_gn, B, 32, 2), torch.float32)
+    gn_scratch = ws.get("gn_scratch", (4 << 20,), torch.uint8, zero=True)     # the kernel leaves it zeroed
+    stat_i = iter(range(n_gn))
+    # fused statistics: the conv epilogue writes per-warp partial sums here (largest layer:
+    # stage 0 at 96x96 -> 72 tiles x 4 quadrants x 32 groups x 2 per image)
+    gn_part = buf("gn_partial", (B * ((H // 4) * (W // 4) // 32 + 64) * 4 * 32 * 2,), torch.float32)
+
+    def conv_stats(fn, *args, out, **kw):
+        """conv + GroupNorm statistics of its (unrounded) output.  Tensor-core path: partial sums in the conv
+        epilogue + finalize; fp32 mode: the deterministic standalone statistics kernel."""
+        st = stats_pool[next(stat_i)]
+        if fp32:
+            fn(*args, out, **kw)
+            ops.groupnorm_stats(out, st, scratch=gn_scratch)
+        else:
+            fn(*args, out, gn_stats=(gn_part, st), **kw)
+        return st
+
+    cols = buf("stem_cols", (B * h2 * w2, 160))
+    ops.stem_im2col(x, cols)
+    s0 = buf("stem_conv", (B, h2, w2, 64))
+    st = conv_stats(ops.conv1x1, cols.view(B, h2, w2, 160), pk["stem_w"], out=s0)
+    t = buf("stem_pool", (B, h2 // 2, w2 // 2, 64))
+    ops.stem_gn_relu_maxpool(s0, st, pk["stem_g"], pk["stem_b"], t)
+    if taps is not None:
+        taps["stem_conv"], taps["stem_pool"] = s0, t
+    if save is not None:
+        save["stem"], save["blocks"] = (cols, s0, st, t), []
+    feats = []
+    hh, ww = h2 // 2, w2 // 2
+    for s, b, e in pk["rn_blocks"]:
+        stride, cout, mid = e["stride"], e["cout"], e["mid"]
+        ho, wo = hh // stride, ww // stride
+        tag = f"s{s}b{b}"
+        shortcut, sc_stats = t, None
+        if b == 0:
+            d = buf(tag + "_ds", (B, ho, wo, cout))
+            sc_stats = conv_stats(ops.conv1x1, t[:, ::stride, ::stride, :] if stride > 1 else t, e["wd"], out=d)
+            shortcut = d
+        y1 = buf(tag + "_y1", (B, hh, ww, mid))
+        st1 = conv_stats(ops.conv1x1, t, e["w1"], out=y1)
+        a1 = buf(tag + "_a1", (B, hh, ww, mid))
+        ops.groupnorm_apply(y1, st1, e["g1"], e["b1"], a1, relu=True)
+        y2 = buf(tag + "_y2", (B, ho, wo, mid))
+        if stride == 1:
+            st2 = conv_stats(ops.conv3x3, a1, e["w2"], out=y2)
+        else:
+            st2 = conv_stats(lambda a, w_, o, **kw: ops.conv3x3_s2(a, w_, o, "same", **kw), a1, e["w2"], out=y2)
+        a2 = buf(tag + "_a2", (B, ho, wo, mid))
+        ops.groupnorm_apply(y2, st2, e["g2"], e["b2"], a2, relu=True)
+        y3 = buf(tag + "_y3", (B, ho, wo, cout))
+        st3 = conv_stats(ops.conv1x1, a2, e["w3"], out=y3)
+        out = buf(tag + "_out", (B, ho, wo, cout))
+        if b == 0:
+            ops.groupnorm_apply(y3, st3, e["g3"], e["b3"], out, relu=True, res=shortcut,
+                                res_stats=sc_stats, res_gamma=e["gd"], res_beta=e["bd"])
+        else:
+            ops.groupnorm_apply(y3, st3, e["g3"], e["b3"], out, relu=True, res=shortcut)
+        if save is not None:
+            rec = dict(tag=tag, p=f"pretrained.model.patch_embed.backbone.stages.{s}.blocks.{b}.", stride=stride, t_in=t,
+                       b=b, s=s, y1=y1, st1=st1, a1=a1, y2=y2, st2=st2, a2=a2, y3=y3, st3=st3, out=out)
+            if b == 0:
+                rec.update(d=shortcut, std=sc_stats)
+            save["blocks"].append(rec)
+        t, hh, ww = out, ho, wo
+        if taps is not None:
+            taps[f"{tag}_out"] = out
+        if b == _STAGES[s][1] - 1:
+            feats.append(t)
+    return feats
+
+
+def network_forward(pk: dict, x: torch.Tensor, ws: _Workspace, arch: dict, fp32: bool, pos, non_negative: bool,
+                    taps: Optional[dict] = None, save: Optional[dict] = None) -> torch.Tensor:
+    """One forward of the network: packed weights `pk` (the structure of `DPTDepthModel._prepack`), input x fp32
+    [B,3,H,W], activation buffers from `ws`, `arch` an `_ARCH` entry, `fp32` the correctness mode, pos = (pos0 fp32
+    [D], pos[1:] fp32 [B, gh*gw, D]).  Returns the output buffer [B,C,H,W] fp32 of `ws`.
+
+    `taps` receives named intermediate activations (tests).  With `save` (DPT-Hybrid only) this is the train-mode
+    forward: every activation the backward of omnidata_b200.train reads gets a buffer of its own and is recorded in
+    `save`; the MLP GELU, the readout GELU and the head tail keep their inputs."""
+    if save is not None and not arch["hybrid"]:
+        raise NotImplementedError("the train-mode forward is built for the DPT-Hybrid model (vitb_rn50_384)")
+    B, _, H, W = x.shape
+    f32 = torch.float32
+    adt = f32 if fp32 else torch.bfloat16                       # activation storage type
+    buf = lambda name, shape, dtype=adt: ws.get(name, shape, dtype)
+    if save is not None:
+        save.update(x=x, B=B, H=H, W=W)
+
+    D, heads = arch["embed"], arch["heads"]
+    hooks = arch["hooks"]
+    if arch["hybrid"]:
+        layer_1, layer_2, f3 = _resnet_features(pk, x, ws, fp32, taps, save)
+        gh, gw = f3.shape[1], f3.shape[2]
+    else:
+        gh, gw = H // 16, W // 16
+    ntok = gh * gw + 1
+    rows = B * ntok
+    if save is not None:
+        save.update(gh=gh, gw=gw, ntok=ntok, f3=f3)
+
+    # ---------------- tokens: patch proj + cls + pos (vit.py:131-147).  The residual stream is fp32 in BOTH
+    # precisions (timm Block.forward adds every branch to an fp32 `x`; SURVEY.md C.1): the proj / fc2 epilogues
+    # read and write fp32, LayerNorm reads fp32.
+    pos0, pos_b = pos
+    if save is None:
+        # the residual stream lives in one buffer per hooked block: the block after a hook writes its first
+        # residual add into the next buffer, which leaves the hooked activation intact
+        tok_bufs = [buf(f"tok_{i}", (B, ntok, D), f32) for i in range(len(hooks))]
+        tok = tok_bufs[0]
+    else:
+        # the stream before every block (xs) and between its two residual adds (xm)
+        xs = [buf(f"vit_x{i}", (B, ntok, D), f32) for i in range(len(pk["vit"]) + 1)]
+        xm = [buf(f"vit_m{i}", (B, ntok, D), f32) for i in range(len(pk["vit"]))]
+        tok = xs[0]
+    ops.write_cls_row(tok, pk["cls"], pos0)
+    if arch["hybrid"]:
+        ops.linear(f3.view(B, 1, gh * gw, 1024), pk["proj_w"], tok[:, 1:, :].unsqueeze(1), bias=pk["proj_b"],
+                   residual=pos_b.unsqueeze(1))
+    else:
+        cols = buf("patch_cols", (B, 1, gh * gw, 3 * 16 * 16))
+        ops.patchify(x, cols.view(B * gh * gw, -1), 16)
+        ops.linear(cols, pk["proj_w"], tok[:, 1:, :].unsqueeze(1), bias=pk["proj_b"], residual=pos_b.unsqueeze(1))
+
+    if taps is not None:
+        taps["tokens_in"] = tok.clone()
+    # ---------------- ViT blocks (vit.py:150-151); final norm is dead compute and skipped
+    if save is None:                                   # scratch shared by all blocks
+        h1 = h2 = buf("vit_h", (B, ntok, D))
+        qkv = buf("vit_qkv", (B, ntok, 3 * D))
+        att = buf("vit_att", (B, ntok, D))
+        mlp = buf("vit_mlp", (B, ntok, 4 * D))
+        lse = None
+    else:
+        vit = []
+    cur = tok
+    hooked = []
+    for i, blk in enumerate(pk["vit"]):
+        if save is None:
+            x_in = cur
+            x_mid = x_out = tok_bufs[len(hooked)] if (i - 1) in hooks else cur
+        else:
+            x_in, x_mid, x_out = xs[i], xm[i], xs[i + 1]
+            h1, h2 = buf(f"vit_h1_{i}", (B, ntok, D)), buf(f"vit_h2_{i}", (B, ntok, D))
+            qkv = buf(f"vit_qkv_{i}", (B, ntok, 3 * D))
+            att = buf(f"vit_att_{i}", (B, ntok, D))
+            lse = None if fp32 else buf(f"vit_lse_{i}", (B, heads, ntok), f32)
+            u, mlp = buf(f"vit_u_{i}", (B, ntok, 4 * D)), buf(f"vit_mlp_{i}", (B, ntok, 4 * D))
+        ops.layernorm(x_in, blk["ln1"][0], blk["ln1"][1], h1)
+        ops.linear(h1.view(rows, -1), blk["qkv"][0], qkv.view(rows, -1), bias=blk["qkv"][1])
+        ops.attention(qkv, att, heads=heads, scale=0.125, lse=lse)
+        ops.linear(att.view(rows, -1), blk["proj"][0], x_mid.view(rows, -1), bias=blk["proj"][1],
+                   residual=x_in.view(rows, -1))
+        ops.layernorm(x_mid, blk["ln2"][0], blk["ln2"][1], h2)
+        if save is None:
+            ops.linear(h2.view(rows, -1), blk["fc1"][0], mlp.view(rows, -1), bias=blk["fc1"][1], act=ops.ACT_GELU)
+        elif fp32:                                     # the fp32 conv kernel has no GELU out2
+            ops.linear(h2.view(rows, -1), blk["fc1"][0], u.view(rows, -1), bias=blk["fc1"][1])
+            bwd.gelu_fwd(u, mlp)
+        else:       # one pass: the pre-activation (kept for the backward) and gelu of the same fp32 value
+            ops.linear(h2.view(rows, -1), blk["fc1"][0], u.view(rows, -1), bias=blk["fc1"][1],
+                       out2=mlp.view(rows, -1), out2_act=ops.ACT_GELU)
+        ops.linear(mlp.view(rows, -1), blk["fc2"][0], x_out.view(rows, -1), bias=blk["fc2"][1],
+                   residual=x_mid.view(rows, -1))
+        cur = x_out
+        if i in hooks:
+            hooked.append(cur)
+        if save is not None:
+            vit.append(dict(h1=h1, qkv=qkv, att=att, lse=lse, h2=h2, u=u, mlp=mlp))
+        if taps is not None:
+            taps[f"tokens_{i}"] = cur.clone()
+    if save is not None:
+        save.update(xs=xs, xm=xm, vit=vit)
+
+    # ---------------- reassemble (vit.py:66-97, 185-290 / 431-462); outputs carried zero-padded to the GEMM's N
+    # granularity
+    def readout(tk32, n):
+        tk = tk32
+        if not fp32:                                   # the hooked activation leaves the fp32 stream as a bf16 operand
+            tk = buf(f"ro{n}_tok", (B, ntok, D))
+            ops.cast_f32_bf16(tk32, tk)
+        cb = buf(f"ro{n}_cb", (B, D), f32)
+        ops.readout_cls_bias(pk[f"ro{n}_wfull"], pk[f"ro{n}_b"], tk, cb)
+        r = buf(f"ro{n}_r", (B, 1, gh * gw, D))
+        if save is None:
+            ops.linear(tk[:, 1:, :].unsqueeze(1), pk[f"ro{n}_wtok"], r, bias=cb, bias_per_image=True, act=ops.ACT_GELU)
+        else:
+            pre = buf(f"ro{n}_pre", (B, 1, gh * gw, D))
+            ops.linear(tk[:, 1:, :].unsqueeze(1), pk[f"ro{n}_wtok"], pre, bias=cb, bias_per_image=True)
+            bwd.gelu_fwd(pre, r)
+        w, bias = pk[f"pp{n}_w"], pk[f"pp{n}_b"]
+        o = buf(f"pp{n}", (B, gh, gw, w.shape[0]))
+        ops.conv1x1(r.view(B, gh, gw, D), w, o, bias=bias)
+        if save is not None:
+            save[f"ro{n}"] = dict(tk=tk, tk32=tk32, pre=pre, r=r, o=o)
         return o
+
+    def conv_transpose(t, n, k):
+        """ConvTranspose2d(c, c, k, stride k): phase (dy, dx) of the output is a 1x1 convolution of the
+        input, stored through a strided view of the output (no scatter kernel)."""
+        c = t.shape[3]
+        o = buf(f"pp{n}t", (B, gh * k, gw * k, c))
+        for dy in range(k):
+            for dx in range(k):
+                ops.conv1x1(t, pk[f"pp{n}t_w"][dy][dx], o[:, dy::k, dx::k, :], bias=pk[f"pp{n}t_b"])
+        return o
+
+    if arch["hybrid"]:
+        tokens_8, tokens_11 = hooked
+        layer_3 = readout(tokens_8, 3)
+        u4 = readout(tokens_11, 4)
+    else:
+        layer_1 = conv_transpose(readout(hooked[0], 1), 1, 4)
+        layer_2 = conv_transpose(readout(hooked[1], 2), 2, 2)
+        layer_3 = readout(hooked[2], 3)
+        u4 = readout(hooked[3], 4)
+    layer_4 = buf("pp4s", (B, gh // 2, gw // 2, pk["pp4s_w"].shape[0]))
+    ops.conv3x3_s2(u4, pk["pp4s_w"], layer_4, "sym1", bias=pk["pp4s_b"])
+
+    # ---------------- scratch.layerN_rn (dpt_depth.py:73-76): raw + relu copies feed the RCUs
+    rn_raw, rn_relu = [], []
+    for n, l in zip((1, 2, 3, 4), (layer_1, layer_2, layer_3, layer_4)):
+        shp = (B, l.shape[1], l.shape[2], _FEATURES)
+        raw, rl = buf(f"rn{n}_raw", shp), buf(f"rn{n}_relu", shp)
+        ops.conv3x3(l, pk[f"rn{n}_w"], raw, out2=rl)
+        rn_raw.append(raw)
+        rn_relu.append(rl)
+    if save is not None:
+        save.update(layers=(layer_1, layer_2, layer_3, layer_4), rn_raw=rn_raw, rn_relu=rn_relu)
+
+    # ---------------- RefineNet fusion (dpt_depth.py:78-81; blocks.py:263-341)
+    def rcu(n, u, x_raw, x_relu, out, out2=None):
+        (w1, b1), (w2, b2) = pk[f"ff{n}_rcu{u}"]
+        tmid = buf(f"ff{n}_rcu{u}_t", x_raw.shape)
+        ops.conv3x3(x_relu, w1, tmid, bias=b1, act=ops.ACT_RELU)       # relu(conv1(relu(x)))
+        ops.conv3x3(tmid, w2, out, bias=b2, residual=x_raw, out2=out2)  # conv2(.) + x
+        if save is not None:
+            save[f"ff{n}.rcu{u}"] = dict(x_raw=x_raw, x_relu=x_relu, tmid=tmid)
+
+    def fusion_tail(n, s_raw, s_relu):
+        """RCU2, then the 1x1 out_conv at the input resolution (it commutes with the bilinear
+        upsample: the interpolation weights sum to one)."""
+        y = buf(f"ff{n}_y", s_raw.shape)
+        rcu(n, 2, s_raw, s_relu, y)
+        z = buf(f"ff{n}_z", s_raw.shape)
+        w, bias = pk[f"ff{n}_out"]
+        ops.conv1x1(y, w, z, bias=bias)
+        if save is not None:
+            save[f"ff{n}"] = dict(y=y, z=z)
+        return z
+
+    z = fusion_tail(4, rn_raw[3], rn_relu[3])
+    if taps is not None:
+        taps["path_4"] = _debug_upsample(z)
+    for n in (3, 2, 1):
+        l_raw, l_relu = rn_raw[n - 1], rn_relu[n - 1]
+        res = buf(f"ff{n}_res", l_raw.shape)
+        rcu(n, 1, l_raw, l_relu, res)
+        s_raw, s_relu = buf(f"ff{n}_s", l_raw.shape), buf(f"ff{n}_s_relu", l_raw.shape)
+        ops.upsample2x_add(z, s_raw, res=res, out_relu=s_relu)         # up(path) + RCU1(layer_rn)
+        z = fusion_tail(n, s_raw, s_relu)
+        if taps is not None and n > 1:
+            taps[f"path_{n}"] = _debug_upsample(z)
+    path_1 = buf("path_1", (B, z.shape[1] * 2, z.shape[2] * 2, _FEATURES))
+    ops.upsample2x_add(z, path_1)
+
+    # ---------------- head (dpt_depth.py:91-99)
+    w0, b0 = pk["head0"]
+    h1 = buf("head_h1", (B, path_1.shape[1], path_1.shape[2], _FEATURES // 2))
+    ops.conv3x3(path_1, w0, h1, bias=b0)
+    h1u = buf("head_h1u", (B, H, W, _FEATURES // 2))
+    ops.upsample2x_add(h1, h1u)
+    w2, b2 = pk["head2"]
+    w4, b4 = pk["head4"]
+    out = buf("out", (B, w4.shape[0], H, W), f32)
+    if save is None and not fp32:
+        ops.conv3x3(h1u, w2, None, bias=b2, head=(w4, b4, out, non_negative))
+    else:
+        # the 128 -> 32 conv (+ReLU) on its own (training: carried zero-padded to 64 channels), then the 1x1 conv
+        # (+ReLU) to NCHW
+        h2 = buf("head_h2", (B, H, W, w2.shape[0]))
+        ops.conv3x3(h1u, w2, h2, bias=b2, act=ops.ACT_RELU)
+        if save is not None:
+            bwd.head_tail_fwd(h2, w4, b4, out, non_negative)
+            save["head"] = dict(path_1=path_1, h1=h1, h1u=h1u, a=h2, out=out, w4=w4)
+        else:
+            pre = buf("head_pre", (B, w4.shape[0], H, W), f32) if taps is not None else None
+            ops.head_tail_f32(h2, w4, b4, out, relu=non_negative, pre=pre)
+            if taps is not None:
+                taps["head_pre_relu"] = pre
+
+    if taps is not None:
+        for hk, tk in zip(hooks, hooked):
+            taps[f"tokens_{hk}"] = tk
+        taps.update(layer_1=layer_1, layer_2=layer_2, layer_3=layer_3, layer_4=layer_4, path_1=path_1,
+                    layer_1_rn=rn_raw[0], layer_2_rn=rn_raw[1], layer_3_rn=rn_raw[2],
+                    layer_4_rn=rn_raw[3])
+    return out

@@ -3,7 +3,8 @@
 
 `TrainEngine(model)` owns flat fp32 parameter / gradient buffers (the model's nn.Parameters become views), re-packs the
 GEMM operands from the fp32 master weights every step (odb_pack_weight: cast, ResNetV2 weight standardisation, dgrad
-layout), runs the forward keeping every activation the backward needs, and the backward:
+layout), runs the model's forward (`model.network_forward`, the one inference runs) with every activation the backward
+needs kept, and the backward:
   * dgrad of every conv / linear layer = odb_conv_gemm with the re-packed (in/out swapped, 180-degree rotated) weight;
     stride-2 convolutions scatter through parity-plane output views;
   * wgrad = odb_conv_wgrad (tcgen05, both operands MN-major straight from the channels-last tensors; fp32 twin);
@@ -22,9 +23,7 @@ import torch
 
 from . import bwd, ops
 from ._capi import OdbError
-from .model import _STAGES, DPTDepthModel
-
-_FEATURES = 256
+from .model import _STAGES, DPTDepthModel, _Workspace, network_forward
 
 
 def _parity_dgrad_plan(mode: str):
@@ -51,7 +50,6 @@ class TrainEngine:
             raise ValueError("precision must be 'bf16' or 'fp32'")
         self.model = model
         self.fp32 = precision == "fp32"
-        self.fuse_gelu = True      # mlp.fc1 writes the pre-activation and its GELU in one epilogue (tensor-core path)
         self.adt = torch.float32 if self.fp32 else torch.bfloat16
         p0 = next(model.parameters())
         if not p0.is_cuda:
@@ -75,18 +73,10 @@ class TrainEngine:
                 self.G[name] = self.flat_grad[off:off + p.numel()].view_as(p.data)
                 off += n
         self.param_names = list(names)
-        self.bufs: Dict[str, torch.Tensor] = {}
-        self._shape = None
+        self.ws = _Workspace(self.device)          # weight operands, activations and gradients
         self._build_layer_table()
+        self.pk = self._packed_weights()
         self.saved = None
-
-    # ------------------------------------------------------------------ buffers
-    def buf(self, name: str, shape, dtype=None) -> torch.Tensor:
-        dtype = self.adt if dtype is None else dtype
-        t = self.bufs.get(name)
-        if t is None or tuple(t.shape) != tuple(shape) or t.dtype != dtype:
-            t = self.bufs[name] = torch.empty(tuple(shape), device=self.device, dtype=dtype)
-        return t
 
     # ------------------------------------------------------------------ weight table / per-step packing
     def _build_layer_table(self):
@@ -151,31 +141,71 @@ class TrainEngine:
         self.zb = torch.zeros(4096, device=self.device, dtype=torch.float32)               # zero "bias" of the dgrad convs:
         #   selects the straight-line (bias / bias + residual) epilogues of the tensor-core kernel
 
+    def _packed_weights(self) -> dict:
+        """The forward's weights, in the structure of DPTDepthModel._prepack, over the engine's persistent operands: the
+        forward GEMM operands of the layer table, views of the fp32 master parameters and the buffers pack() fills."""
+        P, W, get = self.P, {k: w[0] for k, w in self.W.items()}, self.ws.get
+        pm, bb = "pretrained.model.", "pretrained.model.patch_embed.backbone."
+        pk = {"stem_w": get("w.stem", (64, 160), self.adt),
+              "stem_g": P[bb + "stem.norm.weight"], "stem_b": P[bb + "stem.norm.bias"], "rn_blocks": []}
+        for s, (cout, depth) in enumerate(_STAGES):
+            for b in range(depth):
+                p, tag = f"{bb}stages.{s}.blocks.{b}.", f"s{s}b{b}"
+                e = {"stride": 2 if (b == 0 and s > 0) else 1, "cout": cout, "mid": cout // 4}
+                if b == 0:
+                    e.update(wd=W[tag + ".wd"], gd=P[p + "downsample.norm.weight"], bd=P[p + "downsample.norm.bias"])
+                for i in (1, 2, 3):
+                    e[f"w{i}"], e[f"g{i}"], e[f"b{i}"] = W[f"{tag}.w{i}"], P[p + f"norm{i}.weight"], P[p + f"norm{i}.bias"]
+                pk["rn_blocks"].append((s, b, e))
+        pk["proj_w"], pk["proj_b"] = W["proj"], P[pm + "patch_embed.proj.bias"]
+        pk["cls"], pk["pos"] = P[pm + "cls_token"].reshape(-1), P[pm + "pos_embed"]
+        pk["vit"] = []
+        for i in range(12):
+            p = f"{pm}blocks.{i}."
+            pk["vit"].append({"ln1": (P[p + "norm1.weight"], P[p + "norm1.bias"]),
+                              "qkv": (W[f"blk{i}.qkv"], P[p + "attn.qkv.bias"]),
+                              "proj": (W[f"blk{i}.proj"], P[p + "attn.proj.bias"]),
+                              "ln2": (P[p + "norm2.weight"], P[p + "norm2.bias"]),
+                              "fc1": (W[f"blk{i}.fc1"], P[p + "mlp.fc1.bias"]),
+                              "fc2": (W[f"blk{i}.fc2"], P[p + "mlp.fc2.bias"])})
+        for n in (3, 4):
+            p = f"pretrained.act_postprocess{n}."
+            pk[f"ro{n}_wfull"] = get(f"w.ro{n}.full", (768, 1536), self.adt)
+            pk[f"ro{n}_wtok"] = get(f"w.ro{n}.tok", (768, 768), self.adt)
+            pk[f"ro{n}_b"] = P[p + "0.project.0.bias"]
+            pk[f"pp{n}_w"], pk[f"pp{n}_b"] = W[f"pp{n}"], P[p + "3.bias"]
+        pk["pp4s_w"], pk["pp4s_b"] = W["pp4s"], P["pretrained.act_postprocess4.4.bias"]
+        for n in (1, 2, 3, 4):
+            p = f"scratch.refinenet{n}."
+            pk[f"rn{n}_w"] = W[f"rn{n}"]
+            pk[f"ff{n}_out"] = (W[f"ff{n}.out"], P[p + "out_conv.bias"])
+            for u in ((2,) if n == 4 else (1, 2)):
+                pk[f"ff{n}_rcu{u}"] = tuple((W[f"ff{n}.rcu{u}.c{cv}"], P[f"{p}resConfUnit{u}.conv{cv}.bias"]) for cv in (1, 2))
+        pk["head0"] = (W["head0"], P["scratch.output_conv.0.bias"])
+        pk["head2"] = (W["head2"], get("w.head2.bias", (64,), torch.float32))        # zero-padded to 64 like the weight
+        pk["head4"] = (P["scratch.output_conv.4.weight"].reshape(self.C, 32), P["scratch.output_conv.4.bias"])
+        return pk
+
     @torch.no_grad()
-    def pack(self):
-        """fp32 master weights -> GEMM operands (every step: the optimizer just changed them)."""
+    def pack(self, batch: int):
+        """fp32 master weights -> GEMM operands (every step: the optimizer just changed them).  Returns the position
+        embedding as the forward takes it for `batch` images: (pos0 [D], pos[1:] replicated per image [batch, 576, D])."""
         self.pack_table.run()
-        P = self.P
+        P, pk = self.P, self.pk
         bb = "pretrained.model.patch_embed.backbone."
         # stem 7x7 (3 input channels): [64,3,7,7] -> standardise -> [64, (ky,kx,c)=147] padded to 160 columns
         w = P[bb + "stem.conv.weight"]
         std_, mean = torch.std_mean(w, dim=[1, 2, 3], keepdim=True, unbiased=False)
         ws = ((w - mean) / (std_ + 1e-8)).permute(0, 2, 3, 1).reshape(64, 147)
-        stem = self.buf("w.stem", (64, 160))
-        stem.zero_()
-        stem[:, :147].copy_(ws)
-        self.stem_w = stem
+        pk["stem_w"].zero_()
+        pk["stem_w"][:, :147].copy_(ws)
         # ProjectReadout Linear(1536 -> 768): token half as a GEMM operand (fwd / bwd), whole matrix for the cls kernel
         for n in (3, 4):
             wfull = P[f"pretrained.act_postprocess{n}.0.project.0.weight"]
-            wt = self.buf(f"w.ro{n}.full", (768, 1536))
-            wt.copy_(wfull)
-            tokf = self.buf(f"w.ro{n}.tok", (768, 768))
-            tokf.copy_(wfull[:, :768])
-            tokb = self.buf(f"w.ro{n}.tokT", (768, 768))
-            tokb.copy_(wfull[:, :768].t())
-            clsT = self.buf(f"w.ro{n}.clsT", (768, 768), torch.float32)
-            clsT.copy_(wfull[:, 768:].t())
+            pk[f"ro{n}_wfull"].copy_(wfull)
+            pk[f"ro{n}_wtok"].copy_(wfull[:, :768])
+            self.ws.get(f"w.ro{n}.tokT", (768, 768), self.adt).copy_(wfull[:, :768].t())
+            self.ws.get(f"w.ro{n}.clsT", (768, 768), torch.float32).copy_(wfull[:, 768:].t())
         # stride-2 3x3 convolutions: per-parity-plane dgrad operands cut out of the rotated dgrad weight
         self.plane_w = {}
         for key, mode in (("s1b0.w2", "same"), ("s2b0.w2", "same"), ("pp4s", "sym1")):
@@ -184,6 +214,13 @@ class TrainEngine:
             for plane, taps_ in _parity_dgrad_plan(mode).items():
                 cat = torch.cat([wb[:, (8 - t) * n_pad:(9 - t) * n_pad] for t, _, _ in taps_], dim=1).contiguous()
                 self.plane_w[(key, plane)] = (cat, [(0, dx, dy) for _, dy, dx in taps_])
+        b2 = pk["head2"][1]
+        b2.zero_()
+        b2[:32].copy_(P["scratch.output_conv.2.bias"])
+        pos = P["pretrained.model.pos_embed"]
+        pos_b = self.ws.get("pos_expanded", (batch, pos.shape[1] - 1, pos.shape[2]), torch.float32)
+        pos_b.copy_(pos[0, 1:].unsqueeze(0).expand(batch, -1, -1))
+        return pos[0, 0], pos_b
 
     # ------------------------------------------------------------------ small helpers
     def _wgrad(self, key: str, views, taps, dy, n_rows: Optional[int] = None):
@@ -200,28 +237,13 @@ class TrainEngine:
         if n is None or dy.shape[-1] == g.numel():
             bwd.colsum(dy.reshape(-1, dy.shape[-1]), g.view(1, -1))
         else:                                                   # padded output channels (head conv2)
-            tmp = self.buf("tmp.bias", (1, dy.shape[-1]), torch.float32)
+            tmp = self.ws.get("tmp.bias", (1, dy.shape[-1]), torch.float32)
             bwd.colsum(dy.reshape(-1, dy.shape[-1]), tmp)
             g.copy_(tmp[0, :g.numel()])
 
     def _zb(self, w: torch.Tensor):
         """zero bias vector for a dgrad convolution with weight `w` [n_out][K] (tensor-core path only)."""
         return None if self.fp32 else self.zb[: w.shape[0]]
-
-    def _cast(self, name: str, x32: torch.Tensor) -> torch.Tensor:
-        """fp32 residual-stream tensor as a GEMM operand of the activation type."""
-        if self.fp32:
-            return x32
-        t = self.buf(name, x32.shape)
-        ops.cast_f32_bf16(x32, t)
-        return t
-
-    def _conv_stats(self, fn, *args, out, st):
-        if self.fp32:
-            fn(*args, out)
-            ops.groupnorm_stats(out, st, scratch=self.gn_scratch)
-        else:
-            fn(*args, out, gn_stats=(self.gn_part, st))
 
     # ------------------------------------------------------------------ forward (activations kept)
     @torch.no_grad()
@@ -232,193 +254,11 @@ class TrainEngine:
         B, _, H, W = x.shape
         if H % 32 or W % 32 or (H // 16) * (W // 16) + 1 > 640:
             raise ValueError("H and W must be multiples of 32 with at most 639 patches")
-        self.pack()
-        P, Wt, buf = self.P, self.W, self.buf
-        f32 = torch.float32
-        bb = "pretrained.model.patch_embed.backbone."
-        S = self.saved = {"x": x, "B": B, "H": H, "W": W}
-        if "gn_scratch" not in self.bufs:
-            self.bufs["gn_scratch"] = torch.zeros(4 << 20, dtype=torch.uint8, device=self.device)
-        self.gn_scratch = self.bufs["gn_scratch"]
-        self.gn_part = buf("gn_partial", (B * ((H // 4) * (W // 4) // 32 + 64) * 4 * 32 * 2,), f32)
-        n_gn = 1 + sum(3 * d + 1 for _, d in _STAGES)
-        stats = buf("gn_stats", (n_gn, B, 32, 2), f32)
-        si = iter(range(n_gn))
-
-        # ---- ResNetV2 stem
-        h2, w2 = H // 2, W // 2
-        cols = buf("stem_cols", (B * h2 * w2, 160))
-        ops.stem_im2col(x, cols)
-        s0 = buf("stem_conv", (B, h2, w2, 64))
-        st0 = stats[next(si)]
-        self._conv_stats(ops.conv1x1, cols.view(B, h2, w2, 160), self.stem_w, out=s0, st=st0)
-        t = buf("stem_pool", (B, h2 // 2, w2 // 2, 64))
-        ops.stem_gn_relu_maxpool(s0, st0, P[bb + "stem.norm.weight"], P[bb + "stem.norm.bias"], t)
-        S["stem"] = (cols, s0, st0, t)
-        # ---- bottlenecks
-        feats, blocks = [], []
-        hh, ww, cin = h2 // 2, w2 // 2, 64
-        for s, (cout, depth) in enumerate(_STAGES):
-            mid = cout // 4
-            for b in range(depth):
-                p = f"{bb}stages.{s}.blocks.{b}."
-                tag = f"s{s}b{b}"
-                stride = 2 if (b == 0 and s > 0) else 1
-                ho, wo = hh // stride, ww // stride
-                rec = {"tag": tag, "p": p, "stride": stride, "t_in": t, "b": b, "s": s}
-                shortcut, sc_stats = t, None
-                if b == 0:
-                    d = buf(tag + "_ds", (B, ho, wo, cout))
-                    sc_stats = stats[next(si)]
-                    self._conv_stats(ops.conv1x1, t[:, ::stride, ::stride, :] if stride > 1 else t, Wt[tag + ".wd"][0],
-                                     out=d, st=sc_stats)
-                    shortcut = d
-                    rec["d"], rec["std"] = d, sc_stats
-                y1 = buf(tag + "_y1", (B, hh, ww, mid)); st1 = stats[next(si)]
-                self._conv_stats(ops.conv1x1, t, Wt[tag + ".w1"][0], out=y1, st=st1)
-                a1 = buf(tag + "_a1", (B, hh, ww, mid))
-                ops.groupnorm_apply(y1, st1, P[p + "norm1.weight"], P[p + "norm1.bias"], a1, relu=True)
-                y2 = buf(tag + "_y2", (B, ho, wo, mid)); st2 = stats[next(si)]
-                if stride == 1:
-                    self._conv_stats(ops.conv3x3, a1, Wt[tag + ".w2"][0], out=y2, st=st2)
-                else:
-                    self._conv_stats(lambda a, w_, o, **kw: ops.conv3x3_s2(a, w_, o, "same", **kw), a1, Wt[tag + ".w2"][0],
-                                     out=y2, st=st2)
-                a2 = buf(tag + "_a2", (B, ho, wo, mid))
-                ops.groupnorm_apply(y2, st2, P[p + "norm2.weight"], P[p + "norm2.bias"], a2, relu=True)
-                y3 = buf(tag + "_y3", (B, ho, wo, cout)); st3 = stats[next(si)]
-                self._conv_stats(ops.conv1x1, a2, Wt[tag + ".w3"][0], out=y3, st=st3)
-                out = buf(tag + "_out", (B, ho, wo, cout))
-                if b == 0:
-                    ops.groupnorm_apply(y3, st3, P[p + "norm3.weight"], P[p + "norm3.bias"], out, relu=True, res=shortcut,
-                                        res_stats=sc_stats, res_gamma=P[p + "downsample.norm.weight"],
-                                        res_beta=P[p + "downsample.norm.bias"])
-                else:
-                    ops.groupnorm_apply(y3, st3, P[p + "norm3.weight"], P[p + "norm3.bias"], out, relu=True, res=shortcut)
-                rec.update(y1=y1, st1=st1, a1=a1, y2=y2, st2=st2, a2=a2, y3=y3, st3=st3, out=out)
-                blocks.append(rec)
-                t, hh, ww = out, ho, wo
-            feats.append(t)
-            cin = cout
-        S["blocks"] = blocks
-        layer_1, layer_2, f3 = feats
-        gh, gw = f3.shape[1], f3.shape[2]
-        ntok, D, heads = gh * gw + 1, 768, 12
-        rows = B * ntok
-        S.update(gh=gh, gw=gw, ntok=ntok, f3=f3)
-
-        # ---- tokens (fp32 residual stream)
-        pm = "pretrained.model."
-        pos = P[pm + "pos_embed"]
-        if (gh, gw) != (24, 24):
+        if (H // 16, W // 16) != (24, 24):
             raise NotImplementedError("train step: 384x384 inputs (24x24 patch grid)")
-        pos_b = buf("pos_expanded", (B, gh * gw, D), f32)
-        pos_b.copy_(pos[0, 1:].unsqueeze(0).expand(B, -1, -1))
-        xs = [buf(f"vit_x{i}", (B, ntok, D), f32) for i in range(13)]
-        xm = [buf(f"vit_m{i}", (B, ntok, D), f32) for i in range(12)]
-        cls_row = buf("cls_row", (D,), f32)
-        torch.add(P[pm + "cls_token"].reshape(-1), pos[0, 0], out=cls_row)
-        ops.write_cls_row(xs[0], cls_row, torch.zeros_like(cls_row))
-        ops.linear(f3.view(B, 1, gh * gw, 1024), Wt["proj"][0], xs[0][:, 1:, :].unsqueeze(1), bias=P[pm + "patch_embed.proj.bias"],
-                   residual=pos_b.unsqueeze(1))
-        vit = []
-        for i in range(12):
-            p = f"{pm}blocks.{i}."
-            h1 = buf(f"vit_h1_{i}", (B, ntok, D))
-            ops.layernorm(xs[i], P[p + "norm1.weight"], P[p + "norm1.bias"], h1)
-            qkv = buf(f"vit_qkv_{i}", (B, ntok, 3 * D))
-            ops.linear(h1.view(rows, -1), Wt[f"blk{i}.qkv"][0], qkv.view(rows, -1), bias=P[p + "attn.qkv.bias"])
-            att = buf(f"vit_att_{i}", (B, ntok, D))
-            lse = None
-            if not self.fp32:
-                lse = buf(f"vit_lse_{i}", (B, heads, ntok), f32)
-            ops.attention(qkv, att, heads=heads, scale=0.125, lse=lse)
-            ops.linear(att.view(rows, -1), Wt[f"blk{i}.proj"][0], xm[i].view(rows, -1), bias=P[p + "attn.proj.bias"],
-                       residual=xs[i].view(rows, -1))
-            h2_ = buf(f"vit_h2_{i}", (B, ntok, D))
-            ops.layernorm(xm[i], P[p + "norm2.weight"], P[p + "norm2.bias"], h2_)
-            u = buf(f"vit_u_{i}", (B, ntok, 4 * D))
-            mlp = buf(f"vit_mlp_{i}", (B, ntok, 4 * D))
-            if self.fp32 or not self.fuse_gelu:
-                ops.linear(h2_.view(rows, -1), Wt[f"blk{i}.fc1"][0], u.view(rows, -1), bias=P[p + "mlp.fc1.bias"])
-                bwd.gelu_fwd(u, mlp)
-            else:       # one pass: the pre-activation (kept for the backward) and gelu of the same fp32 value
-                ops.linear(h2_.view(rows, -1), Wt[f"blk{i}.fc1"][0], u.view(rows, -1), bias=P[p + "mlp.fc1.bias"],
-                           out2=mlp.view(rows, -1), out2_act=ops.ACT_GELU)
-            ops.linear(mlp.view(rows, -1), Wt[f"blk{i}.fc2"][0], xs[i + 1].view(rows, -1), bias=P[p + "mlp.fc2.bias"],
-                       residual=xm[i].view(rows, -1))
-            vit.append(dict(h1=h1, qkv=qkv, att=att, lse=lse, h2=h2_, u=u, mlp=mlp))
-        S.update(xs=xs, xm=xm, vit=vit)
-
-        # ---- reassemble
-        def readout(tk32, n):
-            tk = self._cast(f"ro{n}_tok", tk32)
-            cb = buf(f"ro{n}_cb", (B, D), f32)
-            ops.readout_cls_bias(self.bufs[f"w.ro{n}.full"], P[f"pretrained.act_postprocess{n}.0.project.0.bias"], tk, cb)
-            pre = buf(f"ro{n}_pre", (B, 1, gh * gw, D))
-            ops.linear(tk[:, 1:, :].unsqueeze(1), self.bufs[f"w.ro{n}.tok"], pre, bias=cb, bias_per_image=True)
-            r = buf(f"ro{n}_r", (B, 1, gh * gw, D))
-            bwd.gelu_fwd(pre, r)
-            o = buf(f"pp{n}", (B, gh, gw, D))
-            ops.conv1x1(r.view(B, gh, gw, D), Wt[f"pp{n}"][0], o, bias=P[f"pretrained.act_postprocess{n}.3.bias"])
-            S[f"ro{n}"] = dict(tk=tk, tk32=tk32, pre=pre, r=r, o=o)
-            return o
-        layer_3 = readout(xs[9], 3)              # hook after block 8
-        u4 = readout(xs[12], 4)                  # hook after block 11
-        layer_4 = buf("pp4s", (B, gh // 2, gw // 2, D))
-        ops.conv3x3_s2(u4, Wt["pp4s"][0], layer_4, "sym1", bias=P["pretrained.act_postprocess4.4.bias"])
-        layers = (layer_1, layer_2, layer_3, layer_4)
-        S["layers"] = layers
-
-        # ---- scratch.layerN_rn
-        rn_raw, rn_relu = [], []
-        for n, l in zip((1, 2, 3, 4), layers):
-            shp = (B, l.shape[1], l.shape[2], _FEATURES)
-            raw, rl = buf(f"rn{n}_raw", shp), buf(f"rn{n}_relu", shp)
-            ops.conv3x3(l, Wt[f"rn{n}"][0], raw, out2=rl)
-            rn_raw.append(raw); rn_relu.append(rl)
-        S.update(rn_raw=rn_raw, rn_relu=rn_relu)
-
-        def rcu(n, u_, x_raw, x_relu, out, out2=None):
-            p = f"scratch.refinenet{n}.resConfUnit{u_}."
-            tmid = buf(f"ff{n}_rcu{u_}_t", x_raw.shape)
-            ops.conv3x3(x_relu, Wt[f"ff{n}.rcu{u_}.c1"][0], tmid, bias=P[p + "conv1.bias"], act=ops.ACT_RELU)
-            ops.conv3x3(tmid, Wt[f"ff{n}.rcu{u_}.c2"][0], out, bias=P[p + "conv2.bias"], residual=x_raw, out2=out2)
-            S[f"ff{n}.rcu{u_}"] = dict(x_raw=x_raw, x_relu=x_relu, tmid=tmid)
-
-        def fusion_tail(n, s_raw, s_relu):
-            y = buf(f"ff{n}_y", s_raw.shape)
-            rcu(n, 2, s_raw, s_relu, y)
-            z = buf(f"ff{n}_z", s_raw.shape)
-            ops.conv1x1(y, Wt[f"ff{n}.out"][0], z, bias=P[f"scratch.refinenet{n}.out_conv.bias"])
-            S[f"ff{n}"] = dict(y=y, z=z)
-            return z
-
-        z = fusion_tail(4, rn_raw[3], rn_relu[3])
-        for n in (3, 2, 1):
-            l_raw, l_relu = rn_raw[n - 1], rn_relu[n - 1]
-            res = buf(f"ff{n}_res", l_raw.shape)
-            rcu(n, 1, l_raw, l_relu, res)
-            s_raw, s_relu = buf(f"ff{n}_s", l_raw.shape), buf(f"ff{n}_s_relu", l_raw.shape)
-            ops.upsample2x_add(z, s_raw, res=res, out_relu=s_relu)
-            z = fusion_tail(n, s_raw, s_relu)
-        path_1 = buf("path_1", (B, z.shape[1] * 2, z.shape[2] * 2, _FEATURES))
-        ops.upsample2x_add(z, path_1)
-        # ---- head (unfused: the backward needs relu(conv2) and the final map)
-        h1 = buf("head_h1", (B, path_1.shape[1], path_1.shape[2], 128))
-        ops.conv3x3(path_1, Wt["head0"][0], h1, bias=P["scratch.output_conv.0.bias"])
-        h1u = buf("head_h1u", (B, H, W, 128))
-        ops.upsample2x_add(h1, h1u)
-        b2 = buf("head_b2pad", (64,), f32)
-        b2.zero_()
-        b2[:32].copy_(P["scratch.output_conv.2.bias"])
-        a = buf("head_a", (B, H, W, 64))
-        ops.conv3x3(h1u, Wt["head2"][0], a, bias=b2, act=ops.ACT_RELU)
-        out = buf("out", (B, self.C, H, W), f32)
-        w4 = P["scratch.output_conv.4.weight"].reshape(self.C, 32)
-        bwd.head_tail_fwd(a, w4, P["scratch.output_conv.4.bias"], out, self.non_negative)
-        S["head"] = dict(path_1=path_1, h1=h1, h1u=h1u, a=a, out=out, w4=w4)
-        return out
+        pos = self.pack(B)
+        self.saved = {}
+        return network_forward(self.pk, x, self.ws, self.model.arch, self.fp32, pos, self.non_negative, save=self.saved)
 
     # ------------------------------------------------------------------ backward
     def _dgrad_s2(self, key: str, dy, dx):
@@ -434,7 +274,8 @@ class TrainEngine:
         on_ready(tag) is called when a contiguous range of the flat gradient is final (plan_grad_buckets): the
         data-parallel train step launches that range's all-reduce while the rest of the backward runs."""
         ready = on_ready if on_ready is not None else (lambda tag: None)
-        S, P, G, Wt, buf = self.saved, self.P, self.G, self.W, self.buf
+        S, P, G, Wt = self.saved, self.P, self.G, self.W
+        buf = lambda name, shape, dtype=self.adt: self.ws.get(name, shape, dtype)
         if S is None:
             raise OdbError("TrainEngine.backward: call forward first")
         B, H, W = S["B"], S["H"], S["W"]
@@ -518,7 +359,7 @@ class TrainEngine:
             self._bias_grad(pp + "3.bias", do)
             bwd.gelu_bwd(dr, r["pre"], dr)
             dtk = buf(f"g.ro{n}_tok", (B, ntok, D))
-            ops.linear(dr, self.bufs[f"w.ro{n}.tokT"], dtk[:, 1:, :].unsqueeze(1))
+            ops.linear(dr, self.ws.get(f"w.ro{n}.tokT", (D, D), self.adt), dtk[:, 1:, :].unsqueeze(1))
             gw_ = G[pp + "0.project.0.weight"]
             gp = self.gp[: D * D].view(D, D)
             bwd.conv_wgrad([r["tk"][:, 1:, :].unsqueeze(1)], bwd.TAPS_1, dr, gp)
@@ -532,7 +373,7 @@ class TrainEngine:
             bwd.conv_wgrad([tok0.view(1, 1, B, D)], bwd.TAPS_1, dcb.view(1, 1, B, D), gp)
             gw_[:, D:].copy_(gp)
             dt0 = buf(f"g.ro{n}_tok0", (B, D), f32)
-            ops.linear(dcb, self.bufs[f"w.ro{n}.clsT"], dt0)
+            ops.linear(dcb, self.ws.get(f"w.ro{n}.clsT", (D, D), f32), dt0)
             dtk[:, 0, :].copy_(dt0)
             return dtk
 
