@@ -85,17 +85,21 @@ def main(argv=None):
     parser.add_argument("--output_path", dest="output_path", help="path to where output image should be stored")
     parser.add_argument("--synthetic_weights", action="store_true")
     parser.add_argument("--weights_dir", default="./pretrained_models/")
+    parser.add_argument("--image_size", type=int, default=384,
+                        help="side of the square network input (a multiple of 32); above 384 gives sharper maps")
     args = parser.parse_args(argv)
     if args.task not in ("normal", "depth"):
         print("task should be one of the following: normal, depth")
         sys.exit()
+    if args.image_size < 32 or args.image_size % 32:
+        parser.error("--image_size must be a positive multiple of 32")
     if not torch.cuda.is_available():
         print("demo.py: a CUDA (sm_100a) device is required; this implementation has no CPU path")
         sys.exit(1)
     device = torch.device("cuda:0")
     os.makedirs(args.output_path, exist_ok=True)
     model = build_model(args.task, args.weights_dir, args.synthetic_weights, device)
-    image_size = 384
+    image_size = args.image_size
     from omnidata_b200 import imageproc
     preprocess = imageproc.DevicePreprocessor(args.task, image_size, device)
 
@@ -105,7 +109,7 @@ def main(argv=None):
             print(f"Reading input {img_path} ...")
             img = Image.open(img_path)
             if img.mode in ("RGB", "L"):
-                # Resize(384, BILINEAR) + CenterCrop + ToTensor [+ Normalize] on the device: the decoded
+                # Resize(image_size, BILINEAR) + CenterCrop + ToTensor [+ Normalize] on the device: the decoded
                 # 8-bit image is uploaded once, the kernels reproduce Pillow's fixed-point resize exactly
                 t = preprocess(np.array(img)).unsqueeze(0)
             else:

@@ -141,12 +141,17 @@ int odb_layernorm(const void* x, const float* gamma, const float* beta, void* y,
 /* Fused multi-head attention (timm Attention.forward): qkv bf16 [b][tokens][3][heads][64] as written
  * by the qkv linear; out bf16 [b][tokens][heads*64]; softmax(q k^T * scale) v.  tcgen05 kernel:
  * S and O accumulate in TMEM, exact two-pass fp32 softmax (global row maximum), P rounded to bf16
- * for the PV product, fp32 row sum of the unrounded P.  tokens <= 640.  lse (optional, training): fp32
- * [b][heads][tokens] = log2 of the row's sum of exp2(s * scale * log2 e), what odb_attention_bwd re-normalises with. */
+ * for the PV product, fp32 row sum of the unrounded P.  Up to 640 tokens all K / V blocks of an (image, head) stay
+ * resident in shared memory; above 640 tokens a second kernel with the same arithmetic streams them through a ring
+ * of shared-memory stages, one work unit per (image, head, 128-query tile).  lse (optional, training, tokens <= 640
+ * only; ODB_ERR_UNSUPPORTED above): fp32 [b][heads][tokens] = log2 of the row's sum of exp2(s * scale * log2 e),
+ * what odb_attention_bwd re-normalises with. */
 int odb_attention(const void* qkv, void* out, float* lse, int32_t b, int32_t tokens, int32_t heads, float scale,
                   void* stream);
 /* fp32 correctness mode of odb_attention: qkv fp32 [b][tokens][3][heads][64], out fp32 [b][tokens][heads*64];
- * dot products and the PV sum in fp64, exp / division exact (no fast-math). */
+ * dot products and the PV sum in fp64, exp / division exact (no fast-math).  Up to 640 tokens a score row is kept
+ * in shared memory; above 640 tokens a kernel with no score buffer makes three passes over the keys (row maximum,
+ * fp64 sum of exp(s - max), PV with s and exp recomputed), with the same definitions. */
 int odb_attention_f32(const float* qkv, float* out, int32_t b, int32_t tokens, int32_t heads, float scale,
                       void* stream);
 

@@ -15,8 +15,8 @@ PKG = Path(__file__).resolve().parent
 CSRC = PKG / "csrc"
 LIB_DIR = PKG / "lib"
 LIB_PATH = LIB_DIR / "libomnidata_b200.so"
-SOURCES = ["api.cu", "conv_gemm.cu", "ops.cu", "attention_tc.cu", "fp32_path.cu", "bwd_ops.cu", "bgemm.cu", "bgemm_tc.cu", "loss.cu",
-           "imageproc.cu", "optim.cu", "refocus.cu"]
+SOURCES = ["api.cu", "conv_gemm.cu", "ops.cu", "attention_tc.cu", "attention_stream.cu", "fp32_path.cu", "bwd_ops.cu",
+           "bgemm.cu", "bgemm_tc.cu", "loss.cu", "imageproc.cu", "optim.cu", "refocus.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-lineinfo", "-std=c++17",
@@ -25,7 +25,7 @@ NVCC_FLAGS = [
 # fast-math (approximate division / sqrt / exp, denormals flushed) only where the arithmetic is bf16-bound anyway:
 # the tensor-core GEMM / attention epilogues and the bf16 elementwise kernels.  The fp32 losses, the optimizer, the
 # fp32 correctness mode, image resampling and the refocus blur promise reference fp32 arithmetic and are built without.
-FAST_MATH_SOURCES = {"conv_gemm.cu", "ops.cu", "attention_tc.cu", "bgemm_tc.cu"}
+FAST_MATH_SOURCES = {"conv_gemm.cu", "ops.cu", "attention_tc.cu", "attention_stream.cu", "bgemm_tc.cu"}
 
 
 def _nvcc() -> str:

@@ -315,6 +315,9 @@ __global__ void __launch_bounds__(kTcThreads, 1) attention_tc_kernel(const __gri
 
 }  // namespace odb
 
+namespace odb { int attention_stream(const void* qkv, void* out, int b, int tokens, int heads, float scale,
+                                     cudaStream_t stream); }   // attention_stream.cu
+
 using namespace odb;
 
 extern "C" int odb_attention(const void* qkv, void* out, float* lse, int32_t b, int32_t tokens, int32_t heads,
@@ -322,8 +325,12 @@ extern "C" int odb_attention(const void* qkv, void* out, float* lse, int32_t b, 
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   if (!qkv || !out || b < 1 || heads < 1 || tokens < 1)
     return fail(ODB_ERR_INVALID, "attention: bad argument");
-  if (tokens > kTcBlk * kTcMaxBlocks) return fail(ODB_ERR_UNSUPPORTED, "attention: at most 640 tokens");
   if (reinterpret_cast<uintptr_t>(qkv) & 15u) return fail(ODB_ERR_INVALID, "attention: qkv must be 16-byte aligned");
+  if (tokens > kTcBlk * kTcMaxBlocks) {
+    // K and V no longer fit in shared memory: they stream through a ring of stages instead
+    if (lse != nullptr) return fail(ODB_ERR_UNSUPPORTED, "attention: lse is only written up to 640 tokens");
+    return attention_stream(qkv, out, b, tokens, heads, scale, stream);
+  }
   AttnTcParams p;
   memset(&p, 0, sizeof(p));
   {

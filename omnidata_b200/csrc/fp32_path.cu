@@ -199,6 +199,92 @@ __global__ void __launch_bounds__(256) attention_f32_kernel(const float* __restr
   }
 }
 
+// Above kAttMaxTok tokens a score row no longer fits in shared memory.  This kernel keeps none: it makes three
+// passes over the keys, kAttKC at a time (K chunk staged in shared memory): the row maximum, the fp64 sum of
+// expf(s - max), then O = P V / l in fp64 with s and the exponential recomputed.  The definitions (fp64 dot
+// products, s = (float)dot * scale, p = expf(s - max), l rounded to fp32) are those of attention_f32_kernel.
+constexpr int kAttKC = 64;
+
+__global__ void __launch_bounds__(256) attention_f32_stream_kernel(const float* __restrict__ qkv,
+                                                                   float* __restrict__ out, int tokens, int heads,
+                                                                   float scale) {
+  __shared__ float q_s[kAttQ][65];
+  __shared__ float k_s[kAttKC][65];
+  __shared__ float s_s[kAttQ][kAttKC];
+  __shared__ float m_s[kAttQ];
+  __shared__ float l_s[kAttQ];
+  const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
+  const int q0 = blockIdx.x * kAttQ, h = blockIdx.y, b = blockIdx.z;
+  const long long row_stride = 3LL * heads * 64;
+  const float* base = qkv + (long long)b * tokens * row_stride + h * 64;
+  for (int i = t; i < kAttQ * 64; i += 256) {
+    const int r = i >> 6, d = i & 63;
+    q_s[r][d] = (q0 + r < tokens) ? base[(long long)(q0 + r) * row_stride + d] : 0.f;
+  }
+  // row reductions: warp w owns rows w and w + 8; PV: thread t owns row t / 16, head dims 4 (t % 16) ..
+  float mx_part[2] = {-INFINITY, -INFINITY};
+  double l_part[2] = {0.0, 0.0};
+  const int r = t >> 4, d4 = (t & 15) * 4;
+  double a0 = 0.0, a1 = 0.0, a2 = 0.0, a3 = 0.0;
+  for (int pass = 0; pass < 3; ++pass) {
+    for (int j0 = 0; j0 < tokens; j0 += kAttKC) {
+      const int nk = tokens - j0 < kAttKC ? tokens - j0 : kAttKC;
+      __syncthreads();                       // the previous chunk is consumed; q_s, m_s and l_s are visible
+      for (int i = t; i < nk * 16; i += 256) {
+        const int jj = i >> 4, dk = (i & 15) * 4;
+        const float4 v = *reinterpret_cast<const float4*>(base + (long long)(j0 + jj) * row_stride + heads * 64 + dk);
+        k_s[jj][dk] = v.x; k_s[jj][dk + 1] = v.y; k_s[jj][dk + 2] = v.z; k_s[jj][dk + 3] = v.w;
+      }
+      __syncthreads();
+      for (int idx = t; idx < kAttQ * nk; idx += 256) {
+        const int rr = idx & (kAttQ - 1), jj = idx / kAttQ;
+        double acc = 0.0;
+#pragma unroll 16
+        for (int d = 0; d < 64; ++d) acc += (double)q_s[rr][d] * (double)k_s[jj][d];
+        s_s[rr][jj] = (float)acc * scale;
+      }
+      __syncthreads();
+      if (pass == 0) {
+#pragma unroll
+        for (int k = 0; k < 2; ++k)
+          for (int jj = lane; jj < nk; jj += 32) mx_part[k] = fmaxf(mx_part[k], s_s[warp + 8 * k][jj]);
+      } else if (pass == 1) {
+#pragma unroll
+        for (int k = 0; k < 2; ++k) {
+          const float m = m_s[warp + 8 * k];
+          for (int jj = lane; jj < nk; jj += 32) l_part[k] += (double)expf(s_s[warp + 8 * k][jj] - m);
+        }
+      } else if (q0 + r < tokens) {
+        const float m = m_s[r];
+        const float* vb = base + 2 * heads * 64 + d4;
+        for (int jj = 0; jj < nk; ++jj) {
+          const double pj = (double)expf(s_s[r][jj] - m);
+          const float4 v = *reinterpret_cast<const float4*>(vb + (long long)(j0 + jj) * row_stride);
+          a0 += pj * (double)v.x; a1 += pj * (double)v.y; a2 += pj * (double)v.z; a3 += pj * (double)v.w;
+        }
+      }
+    }
+#pragma unroll
+    for (int k = 0; k < 2; ++k) {
+      if (pass == 0) {
+        float mx = mx_part[k];
+        for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+        if (lane == 0) m_s[warp + 8 * k] = mx;
+      } else if (pass == 1) {
+        double sum = l_part[k];
+        for (int o = 16; o > 0; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
+        if (lane == 0) l_s[warp + 8 * k] = (float)sum;
+      }
+    }
+  }
+  __syncthreads();
+  if (q0 + r < tokens) {
+    const double inv = 1.0 / (double)l_s[r];
+    float* o = out + ((long long)b * tokens + q0 + r) * (heads * 64) + h * 64 + d4;
+    *reinterpret_cast<float4*>(o) = make_float4((float)(a0 * inv), (float)(a1 * inv), (float)(a2 * inv), (float)(a3 * inv));
+  }
+}
+
 // ------------------------------------------------------------------------------------------ head tail
 __global__ void __launch_bounds__(256) head_tail_f32_kernel(const float* __restrict__ x, const float* __restrict__ w,
                                                             const float* __restrict__ bias, float* __restrict__ out,
@@ -297,11 +383,13 @@ extern "C" int odb_attention_f32(const float* qkv, float* out, int32_t b, int32_
                                  void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   if (!qkv || !out || b < 1 || heads < 1 || tokens < 1) return fail(ODB_ERR_INVALID, "attention_f32: bad argument");
-  if (tokens > kAttMaxTok) return fail(ODB_ERR_UNSUPPORTED, "attention_f32: at most 640 tokens");
   if ((reinterpret_cast<uintptr_t>(qkv) & 15u) || (reinterpret_cast<uintptr_t>(out) & 15u))
     return fail(ODB_ERR_INVALID, "attention_f32: pointers must be 16-byte aligned");
   dim3 grid((tokens + kAttQ - 1) / kAttQ, heads, b);
-  attention_f32_kernel<<<grid, 256, 0, stream>>>(qkv, out, tokens, heads, scale);
+  if (tokens <= kAttMaxTok)
+    attention_f32_kernel<<<grid, 256, 0, stream>>>(qkv, out, tokens, heads, scale);
+  else
+    attention_f32_stream_kernel<<<grid, 256, 0, stream>>>(qkv, out, tokens, heads, scale);
   count_launch();
   return check_launch("attention_f32");
 }

@@ -26,6 +26,7 @@ from ._capi import OdbError
 
 _STAGES = ((256, 3), (512, 4), (1024, 9))   # timm ResNetV2(layers=(3,4,9)) widths / depths
 _FEATURES = 256
+_HYBRID_MAX_W = 1792    # widest input the ResNetV2 stem's im2col kernel stages (odb_stem_im2col)
 # Encoders behind the same decoder (modules/midas/blocks.py:12-47 _make_encoder, dpt_depth.py:41-45 hooks):
 #   vitb_rn50_384  DPT-Hybrid: ResNetV2 stages 0/1 give layer_1/2, ViT-B blocks 8/11 give layer_3/4
 #   vitl16_384     DPT-Large (SURVEY 8(f) rank 3): plain ViT-L/16, blocks 5/11/17/23 give layer_1..4
@@ -408,8 +409,10 @@ class DPTDepthModel(nn.Module):
         if x.dim() != 4 or x.shape[1] != 3:
             raise ValueError(f"expected input [B,3,H,W], got {tuple(x.shape)}")
         B, _, H, W = x.shape
-        if H % 32 or W % 32 or (H // 16) * (W // 16) + 1 > 640:
-            raise ValueError("H and W must be multiples of 32 with at most 639 patches (384x384 in scope)")
+        if H < 32 or W < 32 or H % 32 or W % 32:
+            raise ValueError(f"H and W must be positive multiples of 32, got {H}x{W}")
+        if self.arch["hybrid"] and W > _HYBRID_MAX_W:
+            raise ValueError(f"the hybrid backbone's stem supports input widths up to {_HYBRID_MAX_W}, got {W}")
         if self.training and torch.is_grad_enabled():
             # train() mode under autograd: the differentiable forward (activations kept for the backward kernels);
             # eval() mode, or any call under torch.no_grad(), is the inference path below and returns a tensor
@@ -490,7 +493,10 @@ def _resnet_features(pk, x, ws, fp32, taps, save):
     h2, w2 = H // 2, W // 2
     n_gn = 1 + sum(3 * d + 1 for _, d in _STAGES)
     stats_pool = buf("gn_stats", (n_gn, B, 32, 2), torch.float32)
-    gn_scratch = ws.get("gn_scratch", (4 << 20,), torch.uint8, zero=True)     # the kernel leaves it zeroed
+    # the kernel leaves it zeroed.  The most it needs is for the stem conv (64 channels at H/2) and stage 0's
+    # 256-channel outputs (at H/4), which come to the same size; 4 MiB covers 384x384 up to batch 56
+    gn_need = ops.lib().odb_groupnorm_scratch_bytes(B, h2 * w2, 64, 32)
+    gn_scratch = ws.get("gn_scratch", (max(4 << 20, gn_need),), torch.uint8, zero=True)
     stat_i = iter(range(n_gn))
     # fused statistics: the conv epilogue writes per-warp partial sums here (largest layer:
     # stage 0 at 96x96 -> 72 tiles x 4 quadrants x 32 groups x 2 per image)
